@@ -75,6 +75,9 @@ def parse():
     ap.add_argument("--frozen_dtype", type=str, default=None, help="fp8: E4M3 tensor-core path for the frozen weights (opt-in)")
     ap.add_argument("--attention", type=str, default="auto", choices=["auto", "native", "sdpa"])
     ap.add_argument("--cuda_graphs", type=str, default="true")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="after the timed steps, write what the last step computed (loss, gradient norm, a fixed sample of the "
+                         "parameters) as DIR/<model>_<name>.npy, so that two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -200,6 +203,40 @@ def first_nonfinite(per_rank_log):
     return s, r
 
 
+DUMP_PER_PARAM = 4096  # sampled entries per parameter tensor
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def parameter_sample(model, per_param=DUMP_PER_PARAM, seed=0):
+    """float32 [sum of min(numel, per_param)]: every parameter (module order) at positions drawn from a fixed seed, so the same
+    model configuration always yields the same positions."""
+    import torch
+
+    g = torch.Generator().manual_seed(seed)
+    parts = []
+    for _, p in model.named_parameters():
+        n = p.numel()
+        idx = torch.randint(0, n, (per_param,), generator=g) if n > per_param else torch.arange(n)
+        parts.append(p.detach().flatten()[idx.to(p.device)].float().cpu())
+    return torch.cat(parts)
+
+
+def dump_outputs(out_dir, model_name, loss, grad_norm, model):
+    """The arrays a caller of the training step holds after the last timed step: its loss, the gradient norm of that update and
+    (sampled) the parameters it produced."""
+    import numpy as np
+
+    arrays = {"loss": np.array([float(loss)], dtype=np.float32),
+              "grad_norm": grad_norm.detach().float().reshape(-1).cpu().numpy(),
+              "params_sample": parameter_sample(model).numpy()}
+    nbytes = sum(a.nbytes for a in arrays.values())
+    if nbytes > DUMP_LIMIT_BYTES // 2:  # one half each for the headline model and the llama_1b block
+        raise SystemExit(f"--dump-outputs: {model_name} outputs take {nbytes} bytes, more than {DUMP_LIMIT_BYTES // 2}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{model_name}_{name}.npy"), a)
+
+
 def gather_rows(t):
     """all_gather a 1-D device tensor -> [world, n] on the host."""
     import torch
@@ -240,6 +277,7 @@ def run_ours_case(args, info, model, steps, warmup, rank, local, world):
     loss_log = torch.full((n_log,), float("nan"), dtype=torch.float32, device=dev)   # this rank's loss, before the mean
     norm_log = torch.zeros(n_log, dtype=torch.float32, device=dev)
     cursor = [0]
+    last = {}  # what the most recent step returned to its caller
 
     def record():
         i = cursor[0]
@@ -248,7 +286,7 @@ def run_ours_case(args, info, model, steps, warmup, rank, local, world):
         cursor[0] = i + 1
 
     def dev_step(i):
-        eng.train_step_device(dev_tokens[i])
+        last["loss"] = eng.train_step_device(dev_tokens[i])
         record()
 
     for i in range(warmup):
@@ -271,7 +309,8 @@ def run_ours_case(args, info, model, steps, warmup, rank, local, world):
         losses = []
 
         def e2e_step(i):
-            losses.append(eng.train_step(host[warmup + i]))
+            last["loss"] = eng.train_step(host[warmup + i])
+            losses.append(last["loss"])
             record()
 
         secs2 = timed(e2e_step, steps, world, dev)
@@ -305,6 +344,8 @@ def run_ours_case(args, info, model, steps, warmup, rank, local, world):
             print(f"[bench] NON-FINITE training state ({model}): first bad step {bad_step}, per-rank losses at that step "
                   f"{losses_all[:, bad_step].tolist() if bad_step is not None else None}, norms "
                   f"{norms_all[:, bad_step].tolist() if bad_step is not None else None}", file=sys.stderr)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, last["loss"], eng.last_grad_norm, eng.model)
     # ---- free everything before the next case (graphs, symmetric buffers, activations)
     del eng, dev_tokens, host
     gc.collect()

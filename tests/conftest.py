@@ -1,6 +1,5 @@
 import os
 import sys
-import types
 
 import pytest
 
@@ -11,8 +10,6 @@ if ROOT not in sys.path:
 os.environ.setdefault("RELORA_B200_NO_WANDB", "1")
 os.environ.setdefault("WANDB_MODE", "disabled")
 os.environ.setdefault("TOKENIZERS_PARALLELISM", "false")
-
-REFERENCE = "/root/reference"
 
 
 def pytest_configure(config):
@@ -36,30 +33,3 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip_gpu)
         if "multigpu" in item.keywords and n_gpu < 2:
             item.add_marker(skip_multi)
-
-
-@pytest.fixture(scope="session")
-def reference_modules():
-    """Import the upstream package (read-only mount) with a stub ``bitsandbytes``; skip if absent."""
-    if not os.path.isdir(os.path.join(REFERENCE, "peft_pretraining")):
-        pytest.skip("reference tree not mounted")
-    if "bitsandbytes" not in sys.modules:
-        bnb = types.ModuleType("bitsandbytes")
-        bnb.nn = types.ModuleType("bitsandbytes.nn")
-        bnb.functional = types.ModuleType("bitsandbytes.functional")
-        sys.modules["bitsandbytes"] = bnb
-        sys.modules["bitsandbytes.nn"] = bnb.nn
-        sys.modules["bitsandbytes.functional"] = bnb.functional
-    if REFERENCE not in sys.path:
-        sys.path.append(REFERENCE)
-    try:
-        import importlib
-
-        mods = types.SimpleNamespace(
-            llama=importlib.import_module("peft_pretraining.modeling_llama"),
-            relora=importlib.import_module("peft_pretraining.relora"),
-            training_utils=importlib.import_module("peft_pretraining.training_utils"),
-        )
-    except Exception as e:  # version drift in transformers etc.
-        pytest.skip(f"reference modules not importable here: {type(e).__name__}: {e}")
-    return mods

@@ -52,3 +52,26 @@ def test_both_arms_share_config_keys_and_recipes_follow_the_baseline():
     assert b.RECIPES["llama_250m"]["batch"] * b.RECIPES["llama_250m"]["ga"] * 8 == 1152
     assert b.RECIPES["llama_1b"]["reset"]["optimizer_magnitude_pruning"] == 0.9
     assert b.EXIT_NONFINITE == 3
+
+
+def test_dump_outputs_writes_float_arrays_at_fixed_positions(tmp_path):
+    from relora_b200.models import LlamaForCausalLM, load_config
+
+    b = _bench()
+    torch.manual_seed(0)
+    model = LlamaForCausalLM(load_config(os.path.join(ROOT, "configs", "llama_9m.json")))
+    b.dump_outputs(str(tmp_path / "out"), "llama_9m", 10.5, torch.tensor(0.25), model)
+    names = sorted(os.listdir(tmp_path / "out"))
+    assert names == ["llama_9m_grad_norm.npy", "llama_9m_loss.npy", "llama_9m_params_sample.npy"]
+    import numpy as np
+
+    arrays = {n: np.load(tmp_path / "out" / n) for n in names}
+    assert all(a.dtype == np.float32 for a in arrays.values())
+    assert arrays["llama_9m_loss.npy"].tolist() == [10.5] and arrays["llama_9m_grad_norm.npy"].tolist() == [0.25]
+    want = sum(min(p.numel(), b.DUMP_PER_PARAM) for p in model.parameters())
+    sample = arrays["llama_9m_params_sample.npy"]
+    assert sample.shape == (want,) and sum(a.nbytes for a in arrays.values()) <= b.DUMP_LIMIT_BYTES // 2
+    assert np.array_equal(sample, b.parameter_sample(model).numpy())        # same model, same positions
+    with torch.no_grad():
+        model.lm_head.weight.add_(1.0)
+    assert not np.array_equal(sample, b.parameter_sample(model).numpy())    # the sample sees the parameters

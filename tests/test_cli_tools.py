@@ -22,6 +22,19 @@ def tiny_tokenizer(tmp_path_factory):
     return d
 
 
+@pytest.fixture
+def datasets_cache(tmp_path, monkeypatch):
+    """``datasets.load_dataset`` caches under the user's Hugging Face home, which need not exist or be writable: keep it in
+    the test's own directory."""
+    from datasets import config
+
+    cache = tmp_path / "hf_datasets"
+    monkeypatch.setattr(config, "HF_DATASETS_CACHE", cache)
+    monkeypatch.setattr(config, "DOWNLOADED_DATASETS_PATH", cache / "downloads")
+    monkeypatch.setattr(config, "EXTRACTED_DATASETS_PATH", cache / "downloads" / "extracted")
+    monkeypatch.setattr(config, "HF_MODULES_CACHE", cache / "modules")
+
+
 def _corpus(path, n_lines=400, seed=0):
     import random
 
@@ -31,7 +44,7 @@ def _corpus(path, n_lines=400, seed=0):
             f.write(" ".join(f"w{rng.randrange(200)}" for _ in range(rng.randrange(5, 40))) + "\n")
 
 
-def test_pretokenize_then_train(tiny_tokenizer, tmp_path):
+def test_pretokenize_then_train(tiny_tokenizer, datasets_cache, tmp_path):
     import pretokenize
     from torchrun_main import main as train_main
 
@@ -63,7 +76,7 @@ def test_pretokenize_then_train(tiny_tokenizer, tmp_path):
                     "--save_dir", str(tmp_path / "run2"), "--device", "cpu", "--dtype", "float32", "--workers", "0"])
 
 
-def test_run_glue_on_local_files(tiny_tokenizer, tmp_path):
+def test_run_glue_on_local_files(tiny_tokenizer, datasets_cache, tmp_path):
     import random
 
     import run_glue

@@ -1,65 +1,33 @@
 """Loss-curve parity with the unmodified reference on synthetic tokens (CPU, fp32, llama_9m): same initial weights, same
 batches, the reference's own model / ReLoRaModel / scheduler / optimizer-reset code driven by the loop of
-``torchrun_main.py:768-826`` versus this repo's TrainingEngine (SURVEY.md §4: "reference-vs-new loss-curve parity")."""
+``torchrun_main.py:768-826`` versus this repo's TrainingEngine (SURVEY.md §4: "reference-vs-new loss-curve parity").
+The reference's losses are stored in tests/golden (``tests/reference_golden.py`` regenerates them)."""
 import os
 
-import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-TARGETS = ["attn", "attention", "mlp"]
 
 
-def test_training_losses_match_the_reference_through_a_relora_reset(reference_modules):
-    from transformers import AutoConfig
+def test_training_losses_match_the_reference_through_a_relora_reset():
+    import reference_golden as rg
 
     from relora_b200.engine.api import TrainingEngine
+    from relora_b200.models import load_config
 
-    ref_llama, ref_relora, tu = reference_modules.llama, reference_modules.relora, reference_modules.training_utils
-    steps, relora_every, ga, B, T = 7, 3, 2, 2, 32
-    torch.manual_seed(0)
-    cfg = AutoConfig.from_pretrained("/root/reference/configs/llama_9m.json")
-    ref = ref_llama.LlamaForCausalLM(cfg)
-    ref_w = ref_relora.ReLoRaModel(ref, r=8, lora_alpha=32, target_modules=TARGETS, lora_dropout=0.0, keep_original_weights=True)
-    # make the LoRA branch live from the start (upstream starts with A = B = 0)
-    for mod in ref_w.modules():
-        if isinstance(mod, ref_relora.ReLoRaLinear):
-            torch.nn.init.normal_(mod.lora_A.weight, std=0.02)
-            torch.nn.init.normal_(mod.lora_B.weight, std=0.02)
-
+    c = rg.LOSS_CURVE
+    steps, relora_every, ga, B, T = c["steps"], c["relora_every"], c["ga"], c["B"], c["T"]
+    ref_losses = [float(x) for x in rg.load()["loss_curve:losses"]]
+    assert len(ref_losses) == steps
+    cfg_path = os.path.join(ROOT, "configs", "llama_9m.json")
     eng = TrainingEngine.build(
-        model_config=os.path.join(ROOT, "configs", "llama_9m.json"), batch_size=B, gradient_accumulation=ga, total_batch_size=B * ga,
+        model_config=cfg_path, batch_size=B, gradient_accumulation=ga, total_batch_size=B * ga,
         max_length=T, use_peft=True, lora_r=8, lora_alpha=32, lora_dropout=0.0, relora=relora_every, cycle_length=relora_every,
         scheduler="cosine_restarts", warmup_steps=1, restart_warmup_steps=1, lr=1e-3, num_training_steps=9, dtype="float32", device="cpu",
         reset_optimizer_on_relora=False, optimizer_magnitude_pruning=0.9, clip_grad_norm=1.0, min_lr_ratio=0.1)
-    eng.model.wrapped_model.load_state_dict(ref_w.wrapped_model.state_dict(), strict=True)
-
-    trainable = [p for p in ref_w.parameters() if p.requires_grad]
-    lora_params = [p for n, p in ref_w.named_parameters() if p.requires_grad and "lora_" in n]
-    opt = torch.optim.AdamW(trainable, lr=1e-3, betas=(0.9, 0.999), weight_decay=0.0)
-    sch = tu.get_scheculer(opt, scheduler_type="cosine_restarts", num_training_steps=9, warmup_steps=1, min_lr_ratio=0.1,
-                           cycle_length=relora_every, restart_warmup_steps=1)
-    g = torch.Generator().manual_seed(1)
-    ref_losses, our_losses = [], []
-    ref_w.train()
-    for step in range(1, steps + 1):
-        batch = torch.randint(0, cfg.vocab_size, (ga, B, T), generator=g)
-        tot = 0.0
-        for i in range(ga):
-            loss = ref_w(input_ids=batch[i], labels=batch[i].clone()).loss
-            (loss / ga).backward()
-            tot += float(loss)
-        torch.nn.utils.clip_grad_norm_(trainable, 1.0, error_if_nonfinite=True)
-        opt.step()
-        sch.step()
-        opt.zero_grad()
-        ref_losses.append(tot / ga)
-        our_losses.append(float(eng.train_step(batch)))
-        # upstream resets at update_step % relora == 1 (torchrun_main.py:877-912): merge, then prune the LoRA moments
-        if step % relora_every == 1 and step > 1:
-            ref_w.merge_and_reinit()
-            tu.optimizer_reset(opt, reset_params=lora_params, optimizer_state_keys=["exp_avg", "exp_avg_sq"],
-                               reset_optimizer_on_relora=False, optimizer_random_pruning=0.0, optimizer_magnitude_pruning=0.9)
+    # the reference's weights, with the LoRA branch live from the start (upstream starts with A = B = 0)
+    rg.seed_parameters_(eng.model.wrapped_model)
+    our_losses = [float(eng.train_step(batch)) for batch in rg.loss_curve_batches(load_config(cfg_path).vocab_size)]
     # identical until (and including) the first update after the merge: the merged weights agree and B = 0 on both sides;
     # afterwards the re-initialised A differs by construction (upstream draws it from the torch generator, we hash)
     n_exact = relora_every + 2

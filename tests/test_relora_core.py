@@ -174,34 +174,27 @@ def test_optimizer_reset_modes():
     assert pct > 99
 
 
-def test_reference_relora_state_dict_interchange(reference_modules):
-    """A reference-wrapped model's weights load into ours (and produce the same logits)."""
-    ref_llama, ref_relora = reference_modules.llama, reference_modules.relora
-    from transformers import AutoConfig
+def test_reference_relora_state_dict_interchange():
+    """A reference-wrapped model's weights load into ours (and produce the same logits as the reference, stored in tests/golden)."""
+    import reference_golden as rg
 
-    torch.manual_seed(0)
-    ref_cfg = AutoConfig.from_pretrained(os.path.join("/root/reference/configs", "llama_9m.json"))
-    ref = ref_llama.LlamaForCausalLM(ref_cfg)
-    ref_w = ref_relora.ReLoRaModel(ref, r=8, lora_alpha=32, target_modules=TARGETS, lora_dropout=0.1,
-                                   keep_original_weights=True)
-    for mod in ref_w.modules():
-        if isinstance(mod, ref_relora.ReLoRaLinear):
-            torch.nn.init.normal_(mod.lora_A.weight, std=0.02)
-            torch.nn.init.normal_(mod.lora_B.weight, std=0.02)
+    golden = rg.load()
     ours = ReLoRaModel(_model(), r=8, lora_alpha=32, target_modules=TARGETS)
-    ours.wrapped_model.load_state_dict(ref_w.wrapped_model.state_dict(), strict=True)
-    ref_w.eval(); ours.eval()
-    ids = torch.randint(0, 32000, (2, 24))
+    assert set(ours.wrapped_model.state_dict()) == set(golden["interchange:state_dict_keys"])
+    rg.seed_parameters_(ours.wrapped_model)
+    ours.eval()
+    ids = rg.seeded_ids(**rg.INTERCHANGE_IDS)
     with torch.no_grad():
-        a = ref_w(input_ids=ids, labels=ids)
         b = ours(input_ids=ids, labels=ids)
-    assert torch.allclose(a.logits, b.logits, atol=2e-5)
-    assert abs(float(a.loss) - float(b.loss)) < 1e-5
+    assert torch.allclose(rg.sampled(golden, "interchange:logits", b.logits), torch.from_numpy(golden["interchange:logits"]), atol=2e-5)
+    assert abs(float(golden["interchange:loss"]) - float(b.loss)) < 1e-5
     # merge parity
-    ref_w.merge_and_reinit(); ours.merge_and_reinit()
-    for (n, p), (n2, p2) in zip(ref_w.wrapped_model.named_parameters(), ours.wrapped_model.named_parameters()):
-        if n.endswith("q_proj.weight") or n.endswith("down_proj.weight"):
-            assert torch.allclose(p, p2, atol=1e-6), n
+    ours.merge_and_reinit()
+    merged = [n for n, _ in ours.wrapped_model.named_parameters() if n.endswith("q_proj.weight") or n.endswith("down_proj.weight")]
+    assert len(merged) == 8
+    for n in merged:
+        p2 = ours.wrapped_model.get_parameter(n)
+        assert torch.allclose(rg.sampled(golden, f"interchange:merged:{n}", p2), torch.from_numpy(golden[f"interchange:merged:{n}"]), atol=1e-6), n
 
 
 def test_utils_state_size_lr_alarm_and_packed_bytes():

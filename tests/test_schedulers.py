@@ -72,17 +72,20 @@ def test_validation_errors():
         build_multiplier("nope", num_training_steps=100, warmup_steps=10)
 
 
-def test_matches_reference_everywhere(reference_modules):
-    tu = reference_modules.training_utils
+def test_matches_reference_everywhere():
+    """Every step of both schedules against the reference's lambdas (their values are stored in tests/golden)."""
+    import reference_golden as rg
+
+    golden = rg.load()
     for adjust in (0, 5):
         mine = build_multiplier("cosine_restarts", num_training_steps=200, warmup_steps=20, min_lr_ratio=0.05,
                                 cycle_length=50, restart_warmup_steps=7, adjust_step=adjust)
+        want = golden[f"scheduler:cosine_restarts:adjust{adjust}"]
+        assert len(want) == 200
         for s in range(200):
-            ref = tu._get_cosine_schedule_with_multiple_warmups_lambda(
-                s, num_training_steps=200, first_warmup_steps=20, restart_warmup_steps=7, restart_every=50,
-                min_lr_ratio=0.05, adjust_step=adjust)
-            assert math.isclose(mine(s), ref, rel_tol=1e-12, abs_tol=1e-12), (s, adjust)
+            assert math.isclose(mine(s), float(want[s]), rel_tol=1e-12, abs_tol=1e-12), (s, adjust)
     mine = build_multiplier("cosine", num_training_steps=200, warmup_steps=10, min_lr_ratio=0.1, cycle_length=40)
+    want = golden["scheduler:cosine"]
+    assert len(want) == 200
     for s in range(200):
-        ref = tu._get_cyclical_cosine_schedule_with_min_lr_lambda(s, num_warmup_steps=10, cycle_length=40, min_lr_ratio=0.1)
-        assert math.isclose(mine(s), ref, rel_tol=1e-12, abs_tol=1e-12)
+        assert math.isclose(mine(s), float(want[s]), rel_tol=1e-12, abs_tol=1e-12)
