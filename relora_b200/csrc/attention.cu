@@ -297,12 +297,18 @@ __global__ void __launch_bounds__((4 * kFwdGroups + kFwdGroups) * 32, kFwdGroups
         attn_wait(o_full, (jj - 1) & 1);
         tc_fence_after();
       }
+      // Whether a row moves its reference maximum depends on that row's own scores only.  The TMEM round trip below is
+      // warp-collective, but rows that do not need it keep m and scale by exactly 1, so a row's result never depends on
+      // its warp-mates -- rows of the next batch in a ragged tail tile, or later rows that see later keys.  Rows past T
+      // (next-batch queries loaded into the tail tile) never rescale, so their P may overflow to inf and their O / l turn
+      // inf or NaN.  That is harmless: P·V is row-local (O row r reads only P row r) and those rows are never stored.
+      const bool bump = t < p.T && (mx - m) * p.scale_log2 > 8.0f;
       if (jj == 0) {
         m = mx;  // first step: P·V overwrites O (accumulate = 0), nothing to rescale
-      } else if (__any_sync(0xffffffffu, (mx - m) * p.scale_log2 > 8.0f)) {
-        // rare: bring this warp's rows of O to the new reference maximum
-        const float m_new = fmaxf(m, mx);
-        const float f = fast_exp2((m - m_new) * p.scale_log2);
+      } else if (__any_sync(0xffffffffu, bump)) {
+        // rare: bring the rows that need it to their new reference maximum
+        const float m_new = bump ? mx : m;
+        const float f = bump ? fast_exp2((m - m_new) * p.scale_log2) : 1.0f;
         uint32_t o0[32], o1[32];
         tmem_ld_32x32b_x32(lane_addr + 64, o0);
         tmem_ld_32x32b_x32(lane_addr + 96, o1);

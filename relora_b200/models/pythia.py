@@ -149,8 +149,11 @@ class GPTNeoXAttention(nn.Module):
     def forward(self, hidden_states, attention_mask, position_ids, layer_past=None, use_cache=False):
         B, T, _ = hidden_states.shape
         qkv = self.query_key_value(hidden_states).view(B, T, self.num_attention_heads, 3 * self.head_size)
+        # the native path is plain causal attention: it takes no padding mask, so batched eval with a mask stays on the masked
+        # SDPA branch below (same condition as that branch's unmasked case)
         if (layer_past is None and not use_cache and getattr(position_ids, "_rb_default", False) and _native(qkv)
-                and self.rotary_ndims % 2 == 0 and not self.training_dropout_active()):
+                and self.rotary_ndims % 2 == 0 and not self.training_dropout_active()
+                and (attention_mask is None or B == 1 or self.training)):
             return self._forward_native(qkv, B, T)
         q = qkv[..., : self.head_size].permute(0, 2, 1, 3)
         k = qkv[..., self.head_size : 2 * self.head_size].permute(0, 2, 1, 3)
