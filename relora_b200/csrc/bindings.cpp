@@ -295,12 +295,20 @@ void attention_bwd(const Tensor& qkv, const Tensor& out, const Tensor& dout, con
   rb::attention_bwd(d, cur_stream());
 }
 
+// bf16 cos / sin tables [n_pos, rotary_dim] covering positions pos0 .. pos0 + T - 1 (the kernels read them unchecked)
+void chk_rope_tables(const Tensor& cos, const Tensor& sin, int64_t T, int64_t pos0, int64_t rotary_dim, int64_t hd) {
+  chk_bf16(cos, "cos"); chk_bf16(sin, "sin");
+  TORCH_CHECK(cos.dim() == 2 && cos.is_contiguous() && sin.is_contiguous() && cos.size(1) == rotary_dim && sin.sizes() == cos.sizes(),
+              "cos/sin must be contiguous [n_pos, rotary_dim]");
+  TORCH_CHECK(rotary_dim > 0 && rotary_dim <= hd, "rotary_dim must be in (0, head_dim]");
+  TORCH_CHECK(pos0 >= 0 && T + pos0 <= cos.size(0), "rotary table too short");
+}
+
 void rope_inplace(Tensor& buf, int64_t T, int64_t n_rot_heads, int64_t hd, int64_t rotary_dim, const Tensor& cos, const Tensor& sin,
                   bool backward, int64_t pos0) {
-  chk_bf16(buf, "buf"); chk_bf16(cos, "cos"); chk_bf16(sin, "sin");
+  chk_bf16(buf, "buf");
   chk_2d_rowmajor(buf, "buf");
-  TORCH_CHECK(cos.is_contiguous() && sin.is_contiguous() && cos.size(-1) == rotary_dim, "cos/sin must be [n_pos, rotary_dim]");
-  TORCH_CHECK(T + pos0 <= cos.size(0), "rotary table too short");
+  chk_rope_tables(cos, sin, T, pos0, rotary_dim, hd);
   c10::cuda::CUDAGuard guard(buf.device());
   rb::rope_inplace(buf.data_ptr(), buf.stride(0), (int)buf.size(0), (int)T, (int)n_rot_heads, (int)hd, (int)rotary_dim, cos.data_ptr(),
                    sin.data_ptr(), backward, (int)pos0, cur_stream());
@@ -313,6 +321,7 @@ void rope_pack_bwd(const Tensor& dq, const Tensor& dk, const Tensor& dv, Tensor&
   TORCH_CHECK(dq.strides() == dk.strides() && dq.strides() == dv.strides(), "dq/dk/dv must share strides");
   const int B = (int)dq.size(0), nh = (int)dq.size(1), T = (int)dq.size(2), hd = (int)dq.size(3);
   TORCH_CHECK(out.size(0) == (int64_t)B * T && out.size(1) == 3 * (int64_t)nh * hd, "out must be [B*T, 3*nh*hd]");
+  chk_rope_tables(cos, sin, T, pos0, rotary_dim, hd);
   for (const Tensor* t : {&dq, &dk, &dv}) TORCH_CHECK((reinterpret_cast<uintptr_t>(t->data_ptr()) & 15) == 0, "16-byte alignment required");
   c10::cuda::CUDAGuard guard(out.device());
   rb::rope_pack_bwd(dq.data_ptr(), dk.data_ptr(), dv.data_ptr(), dq.stride(0), dq.stride(1), dq.stride(2), out.data_ptr(), out.stride(0), B, T, nh,

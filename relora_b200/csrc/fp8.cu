@@ -109,7 +109,8 @@ __global__ void prep_kernel(float* __restrict__ state, const float* __restrict__
   if (i >= n) return;
   const float fmax = i < n_e4m3 ? kE4M3Max : 57344.f;  // sites >= n_e4m3 are gradients quantised to E5M2
   const float cur = state[2 * i + 1];
-  const float prev = cur > 0.f ? cur : state[2 * i];  // nothing recorded yet: keep the old estimate
+  // nothing recorded yet, or an overflowed activation (inf; NaN fails the comparison too): keep the old estimate
+  const float prev = (isfinite(cur) && cur > 0.f) ? cur : state[2 * i];
   state[2 * i] = prev;
   state[2 * i + 1] = 0.f;
   const float sx = fmaxf(prev, 1e-12f) * margin / fmax;

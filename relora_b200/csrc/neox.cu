@@ -168,8 +168,9 @@ __device__ __forceinline__ float gelu_tanh(float z) {
   return 0.5f * z * (1.f + tanhf(u));
 }
 __device__ __forceinline__ float dgelu_tanh(float z) {
-  const float u = 0.7978845608028654f * (z + 0.044715f * z * z * z), t = tanhf(u);
-  return 0.5f * (1.f + t) + 0.5f * z * (1.f - t * t) * 0.7978845608028654f * (1.f + 3.f * 0.044715f * z * z);
+  const float u = 0.7978845608028654f * (z + 0.044715f * z * z * z), t = tanhf(u), sech2 = 1.f - t * t;
+  // sech2 is exactly 0 once |u| > 9; skipping the term then keeps 0 * inf (z * z overflows above 1.8e19) from giving NaN
+  return 0.5f * (1.f + t) + (sech2 > 0.f ? 0.5f * z * sech2 * 0.7978845608028654f * (1.f + 3.f * 0.044715f * z * z) : 0.f);
 }
 
 template <bool TANH>
